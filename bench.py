@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native SHAPY hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 64]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 64] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +22,9 @@ cpu_baseline / --impl reference: the CPU restatement of the reference path (orac
          is also the bench's SELF-CHECK: the oracle's vertices / betas / measurements of the sampled images are
          compared with the GPU outputs of the same images before anything is timed ("selfcheck" in the line).
 config2 : BASELINE configs[1] (HRNet-W48 only, plain fp16 operands, B = 32) timed in the same run.
+dump    : --dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, float32 or float64, at
+         most 64 MB (a seeded sample of the batch rows beyond that): two builds can be compared output for output, the
+         inputs being seeded.
 config5 : (N > 1) BASELINE configs[4]: rank 0 holds the whole batch (N x 64 uint8 images) in HBM, NCCL scatter ->
          on-device crop / normalise -> forward -> NCCL gather of vertices / betas / measurements to rank 0.
 """
@@ -42,6 +45,7 @@ LBS_CONST_BYTES = 68.93e6                    # dense SMPL-X constants streamed b
 LBS_BODY_BYTES = 254896                      # per-body compulsory I/O
 SHAPE_CONST_BYTES = 1.38e6
 SHAPE_BODY_BYTES = 40 + 125700
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks():
@@ -123,6 +127,48 @@ def usable_cores() -> int:
     return max(1, min(n, 64))
 
 
+def output_arrays(out, prefix='', seen=None):
+    """{dotted name: host array} of every tensor in a forward's output (`stage_02.vertices`, `measurements.chest`,
+    `camera_parameters.scale`, ...).  float32 / float64 stay as they are, other dtypes become float64 (exact for the
+    integer tables); an object met twice (the measurement dict, faces, proj_joints) is written once."""
+    import numpy as np
+    import torch
+    seen = set() if seen is None else seen
+    if id(out) in seen:
+        return {}
+    seen.add(id(out))
+    if isinstance(out, dict):
+        items = out.items()
+    elif hasattr(out, 'KEYS'):                                              # CameraParams
+        items = ((k, getattr(out, k, None)) for k in out.KEYS)
+    else:
+        a = getattr(out, '_t', out)                                         # KeypointTensor wraps its tensor
+        if torch.is_tensor(a):
+            a = a.detach().cpu().numpy()
+        if not isinstance(a, np.ndarray):
+            return {}
+        return {prefix: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)}
+    arrays = {}
+    for k, v in sorted(items, key=lambda kv: str(kv[0])):
+        arrays.update(output_arrays(v, f'{prefix}.{k}' if prefix else str(k), seen))
+    return arrays
+
+
+def dump_outputs(arrays, batch, path):
+    """Writes `arrays` as path/<name>.npy; above DUMP_LIMIT_BYTES only a seeded sample of the batch rows is written."""
+    import numpy as np
+    per_row = sum(a.nbytes // batch for a in arrays.values() if a.ndim and a.shape[0] == batch)
+    fixed = sum(a.nbytes for a in arrays.values()) - per_row * batch
+    n = min(batch, (DUMP_LIMIT_BYTES - fixed) // max(per_row, 1))
+    if n < batch:
+        rows = np.sort(np.random.default_rng(0).choice(batch, n, replace=False))
+        arrays = {k: a[rows] if a.ndim and a.shape[0] == batch else a for k, a in arrays.items()}
+        print(f'bench: --dump-outputs keeps {n} of {batch} rows', file=sys.stderr)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + '.npy'), a)
+
+
 def cpu_reference_step(sd, smplx, lm, x):
     """One pass of the CPU restatement of the reference path (oracle/) over the images `x`."""
     import torch
@@ -161,8 +207,11 @@ def run_reference(args):
     cpu_reference_step(sd, smplx, lm, x)                                     # warm-up pass at the timed sample size
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_reference_step(sd, smplx, lm, x)
+        out = cpu_reference_step(sd, smplx, lm, x)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        out['measurements'] = {k: torch.tensor([m[k] for m in out['measurements']]) for k in out['measurements'][0]}
+        dump_outputs(output_arrays(out), sample, args.dump_outputs)
     v = sample / dt
     line = {'impl': 'reference', 'metric': METRIC, 'value': v, 'unit': 'bodies/s', 'n_gpus': args.gpus,
             'steps': args.steps, 'warmup': 1, 'ms_per_step': dt * 1e3, 'higher_is_better': True,
@@ -188,7 +237,10 @@ def main():
     ap.add_argument('--mode', type=int, default=1, help='1 = split-fp16 parity mode (1e-4), 0 = plain fp16 (config 2)')
     ap.add_argument('--ref-sample', type=int, default=8)
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -223,9 +275,14 @@ def main():
             dist.barrier()
             torch.cuda.synchronize()
 
+    last = {}
+
     def step_resident():
         with torch.no_grad():
-            return model(x_dev)
+            out = model(x_dev)
+        if args.dump_outputs:
+            last['out'] = out
+        return out
 
     def timed(fn, k, pre=None):
         """Sum of per-step device times (CUDA events on the launching stream), L2 flushed before each step."""
@@ -258,6 +315,8 @@ def main():
     with ClockSampler(local_rank) as clk:
         total_ms = timed(step_resident, K)
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(output_arrays(last.pop('out')), B, args.dump_outputs)
     ms_per_step = total_ms / K
     value = world * B / (ms_per_step * 1e-3)
 

@@ -12,15 +12,6 @@ GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run on the B200 box)')
-    config.addinivalue_line('markers', 'reference: needs /root/reference (build container only)')
-
-
-def pytest_collection_modifyitems(config, items):
-    has_ref = os.path.isdir('/root/reference/regressor/human_shape')
-    skip_ref = pytest.mark.skip(reason='/root/reference not present')
-    for item in items:
-        if 'reference' in item.keywords and not has_ref:
-            item.add_marker(skip_ref)
 
 
 @pytest.fixture(scope='session')

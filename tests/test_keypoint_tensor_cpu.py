@@ -2,11 +2,10 @@
 the mirror class, derived from the reference's class (regressor/human_shape/models/body_models/utils.py:123-309):
 indexing gives the plain tensor, tensor methods and torch functions give a KeypointTensor that keeps the keypoint
 metadata, `numpy()` gives the array, everything else is forwarded to the wrapped tensor."""
-import importlib.util
+import json
 import os
 
 import numpy as np
-import pytest
 import torch
 
 from shapy_b200.human_shape.models.body_models.utils import KeypointTensor
@@ -51,31 +50,27 @@ def test_methods_and_torch_functions_keep_the_metadata():
     assert KeypointTensor.from_obj(torch.zeros(1, 3, 3), k).shape == (1, 3, 3)
 
 
-def _reference_class():
-    path = '/root/reference/regressor/human_shape/models/body_models/utils.py'
-    if not os.path.exists(path):
-        return None
-    src = open(path).read()
-    # only the class: the module's other imports (loguru, yacs ...) are not needed for it
-    start = src.index('class KeypointTensor(object):')
-    end = src.index('\nclass ', start + 10) if '\nclass ' in src[start + 10:] else len(src)
-    ns = {'torch': torch}
-    exec(compile(src[start:end], path, 'exec'), ns)      # executed from where it lies, nothing is copied into the repo
-    return ns['KeypointTensor']
+# tensor METHODS only: the reference's instance-level __torch_function__ predates torch 1.7's protocol and returns
+# NotImplemented under torch 2.x, so torch.* functions on its class cannot be compared
+REFERENCE_OPS = [lambda k: k.view(2, 9), lambda k: k.detach(), lambda k: k.to(torch.float64), lambda k: k.sum(dim=2),
+                 lambda k: k.matmul(torch.full((3, 3), 0.5)), lambda k: k.clone().reshape(3, 6), lambda k: k.permute(2, 0, 1)]
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference'), reason='the reference tree only exists in the build container')
-def test_same_results_as_the_reference_class():
-    Ref = _reference_class()
-    a, b = make(), make(Ref)
-    # tensor METHODS only: the reference's instance-level __torch_function__ predates torch 1.7's protocol and returns
-    # NotImplemented under torch 2.x, so torch.* functions on its class cannot be compared here
-    ops = [lambda k: k.view(2, 9), lambda k: k.detach(), lambda k: k.to(torch.float64), lambda k: k.sum(dim=2),
-           lambda k: k.matmul(torch.full((3, 3), 0.5)), lambda k: k.clone().reshape(3, 6), lambda k: k.permute(2, 0, 1)]
-    for f in ops:
-        x, y = f(a), f(b)
-        assert type(x).__name__ == type(y).__name__ == 'KeypointTensor'
-        assert torch.equal(x._t, y._t) and x.keypoint_names == y.keypoint_names and x.source == y.source
-        assert x.connections == y.connections and x.part_indices == y.part_indices
-    assert torch.equal(a[1], b[1]) and type(a[1]) is type(b[1])
-    assert np.array_equal(a.numpy(), b.numpy())
+def record(k):
+    """What is compared with the reference class: result type, wrapped values and keypoint metadata, as JSON values."""
+    return dict(type=type(k).__name__, dtype=str(k._t.dtype), shape=list(k._t.shape), values=k._t.reshape(-1).tolist(),
+                keypoint_names=k.keypoint_names, source=k.source, connections=[list(c) for c in k.connections],
+                part_indices=k.part_indices)
+
+
+def test_same_results_as_the_reference_class(golden_dir):
+    """The mirror against the reference's own class on REFERENCE_OPS: tests/golden/keypoint_tensor.json holds what the
+    reference class returned (tools/make_golden.py keypoint)."""
+    with open(os.path.join(golden_dir, 'keypoint_tensor.json')) as f:
+        ref = json.load(f)
+    a = make()
+    assert len(ref['ops']) == len(REFERENCE_OPS)
+    for f, r in zip(REFERENCE_OPS, ref['ops']):
+        assert record(f(a)) == r
+    assert a[1].tolist() == ref['index1'] and type(a[1]).__name__ == ref['index1_type']
+    assert a.numpy().tolist() == ref['numpy']

@@ -91,15 +91,14 @@ def _gen_after_first():
     return gen
 
 
-@pytest.mark.reference
-def test_smplx_oracle_vs_live_reference():
-    from oracle import ref_shim
+def test_smplx_oracle_vs_live_reference(golden_dir):
+    """Against SMPLX.forward of the reference re-assembled on its verbatim lbs.py (oracle/ref_shim.py) on a second seeded
+    batch: tests/golden/ref_smplx_seed5.npz (tools/make_golden.py smplx_seed5) stores every 4th vertex."""
+    g = np.load(os.path.join(golden_dir, 'ref_smplx_seed5.npz'))
     model = synth.make_smplx()
-    g = torch.Generator().manual_seed(5)
-    betas = torch.randn(2, 10, generator=g)
-    raw = torch.randn(2, 132, generator=g) * 0.3 + synth.mean_params()[:132]
+    betas, raw = torch.from_numpy(g['betas']), torch.from_numpy(g['raw'])
     grot, bpose = smplx_oracle.decode_6d(raw[:, :6]), smplx_oracle.decode_6d(raw[:, 6:])
-    ref = ref_shim.smplx_forward_ref(model, betas, grot, bpose)
     out = smplx_oracle.smplx_forward(model, betas, grot, bpose)
-    for k in ('vertices', 'joints', 'v_shaped'):
-        assert _rel(out[k].numpy(), ref[k].numpy()) < 2e-6
+    assert _rel(out['vertices'][:, ::4].numpy(), g['vertices_sub']) < 2e-6
+    assert _rel(out['joints'].numpy(), g['joints']) < 2e-6
+    assert _rel(out['v_shaped'][:, ::4].numpy(), g['v_shaped_sub']) < 2e-6

@@ -1,16 +1,12 @@
-"""Output writers (SURVEY.md 8f rank 4): camera conversion against the reference's own function text, .npz contents as
+"""Output writers (SURVEY.md 8f rank 4): camera conversion against the reference's own function, .npz contents as
 demo.py:338-352 builds them, .ply round trip.  Pure host code."""
-import ast
 import os
-from collections import defaultdict
 
 import numpy as np
 import pytest
 import torch
 
 from shapy_b200 import writer
-
-REF_DEMO = '/root/reference/regressor/demo.py'
 
 
 class Target:
@@ -30,22 +26,16 @@ def make_targets(n, rng):
             for i in range(n)]
 
 
-def test_camera_conversion_matches_reference_source():
-    """Executes the text of weak_persp_to_blender from the reference's demo.py (build container only) next to the mirror."""
-    if not os.path.exists(REF_DEMO):
-        pytest.skip('reference tree not mounted')
-    src = open(REF_DEMO).read()
-    fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == 'weak_persp_to_blender'][0]
-    ns = {'torch': torch, 'np': np, 'defaultdict': defaultdict}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), REF_DEMO, 'exec'), ns)
-    rng = np.random.default_rng(2)
-    targets = make_targets(5, rng)
-    scale, transl = torch.rand(5, 1) + 0.5, torch.randn(5, 2) * 0.1
-    ref = ns['weak_persp_to_blender'](targets, scale, transl, H=720, W=1280, sensor_width=36, focal_length=5000)
-    mine = writer.weak_persp_to_blender(targets, scale, transl, H=720, W=1280, sensor_width=36, focal_length=5000)
-    assert sorted(ref) == sorted(mine)
-    for k in ref:
-        assert np.array_equal(np.asarray(ref[k]), np.asarray(mine[k])), k
+def test_camera_conversion_matches_reference_source(golden_dir):
+    """The mirror against the outputs of weak_persp_to_blender of the reference's demo.py on the same targets and camera
+    parameters (tests/golden/camera.npz, written by tools/make_golden.py camera)."""
+    g = np.load(os.path.join(golden_dir, 'camera.npz'))
+    targets = [Target(orig_bbox_size=float(s), orig_center=c) for s, c in zip(g['bbox_size'], g['center'])]
+    mine = writer.weak_persp_to_blender(targets, torch.from_numpy(g['scale']), torch.from_numpy(g['transl']), H=720, W=1280,
+                                        sensor_width=36, focal_length=5000)
+    assert sorted(mine) == sorted(g['keys'].tolist())
+    for k in mine:
+        assert np.array_equal(np.asarray(mine[k]), g[f'out_{k}']), k
 
 
 def test_ply_round_trip(tmp_path):

@@ -23,6 +23,11 @@ Everything written here is a small fixture that travels to the GPU box, where
   v2v.npz               reference PointError(TranslationAlignment / NoAlignment) outputs (`v2v_t` / `v2v`) on two seeded meshes
   preprocess.npz        reference input stage (transf_utils.crop with cv2 + ToTensor + Normalize) on seeded uint8 images:
                         crop windows, crops with OpenCV's portable path (IPP off) and with this container's IPP build
+  ref_smplx_seed5.npz   reference SMPLX.forward on a second seeded batch (every 4th vertex)
+  keypoint_tensor.json  the reference KeypointTensor class through the tensor methods of test_keypoint_tensor_cpu.py
+  camera.npz            the reference weak_persp_to_blender (demo.py) on seeded targets and camera parameters
+  ref_mmi.npz           the reference mesh_to_mesh_forward kernel (oracle/_ref; `python tools/make_golden.py mmi` on a
+                        GPU) on the cases of test_gpu_zz_reference_op.py
 """
 import hashlib
 import json
@@ -312,8 +317,108 @@ def p2p_fixture():
     print('p2p.npz', os.path.getsize(os.path.join(G, 'p2p.npz')), 'bytes; mean aligned error', out['mean_aligned'])
 
 
+def _test_module(name):
+    """tests/<name>.py, whose inputs and helpers the fixtures below share."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location(name, os.path.join(ROOT, 'tests', name + '.py'))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def smplx_seed5_fixture():
+    """ref_shim.smplx_forward_ref on the seed-5 batch of test_oracle_pins.py, the rotations decoded by the oracle's
+    decode_6d as the test does; vertices and v_shaped at every 4th vertex (the file stays small)."""
+    from oracle import smplx_oracle
+    from shapy_b200 import synth
+    model = synth.make_smplx()
+    g = torch.Generator().manual_seed(5)
+    betas = torch.randn(2, 10, generator=g)
+    raw = torch.randn(2, 132, generator=g) * 0.3 + synth.mean_params()[:132]
+    grot, bpose = smplx_oracle.decode_6d(raw[:, :6]), smplx_oracle.decode_6d(raw[:, 6:])
+    ref = ref_shim.smplx_forward_ref(model, betas, grot, bpose)
+    np.savez_compressed(os.path.join(G, 'ref_smplx_seed5.npz'), betas=betas.numpy(), raw=raw.numpy(),
+                        vertices_sub=ref['vertices'][:, ::4].numpy(), joints=ref['joints'].numpy(),
+                        v_shaped_sub=ref['v_shaped'][:, ::4].numpy())
+    print('ref_smplx_seed5.npz', os.path.getsize(os.path.join(G, 'ref_smplx_seed5.npz')), 'bytes')
+
+
+def keypoint_fixture():
+    """Runs the reference's own KeypointTensor (regressor/human_shape/models/body_models/utils.py:123-309; the class text
+    only, executed from where it lies: the module's other imports are not needed for it) through REFERENCE_OPS of
+    test_keypoint_tensor_cpu.py."""
+    t = _test_module('test_keypoint_tensor_cpu')
+    path = os.path.join(ref_shim.HS, 'models', 'body_models', 'utils.py')
+    src = open(path).read()
+    start = src.index('class KeypointTensor(object):')
+    end = src.index('\nclass ', start + 10) if '\nclass ' in src[start + 10:] else len(src)
+    ns = {'torch': torch}
+    exec(compile(src[start:end], path, 'exec'), ns)
+    k = t.make(ns['KeypointTensor'])
+    out = dict(ops=[t.record(f(k)) for f in t.REFERENCE_OPS], index1=k[1].tolist(), index1_type=type(k[1]).__name__,
+               numpy=k.numpy().tolist())
+    with open(os.path.join(G, 'keypoint_tensor.json'), 'w') as f:
+        json.dump(out, f)
+    print('keypoint_tensor.json', [r['type'] for r in out['ops']])
+
+
+def camera_fixture():
+    """Runs weak_persp_to_blender of the reference's regressor/demo.py:70-106 (the function text, executed from where it
+    lies) on seeded targets and weak-perspective camera parameters."""
+    import ast
+    from collections import defaultdict
+    t = _test_module('test_writer_cpu')
+    path = os.path.join(REF, 'regressor', 'demo.py')
+    src = open(path).read()
+    fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == 'weak_persp_to_blender'][0]
+    ns = {'torch': torch, 'np': np, 'defaultdict': defaultdict}
+    exec(compile(ast.Module(body=[fn], type_ignores=[]), path, 'exec'), ns)
+    targets = t.make_targets(5, np.random.default_rng(2))
+    g = torch.Generator().manual_seed(2)
+    scale, transl = torch.rand(5, 1, generator=g) + 0.5, torch.randn(5, 2, generator=g) * 0.1
+    ref = ns['weak_persp_to_blender'](targets, scale, transl, H=720, W=1280, sensor_width=36, focal_length=5000)
+    np.savez_compressed(
+        os.path.join(G, 'camera.npz'), bbox_size=np.array([x.get_field('orig_bbox_size') for x in targets]),
+        center=np.stack([x.get_field('orig_center') for x in targets]), scale=scale.numpy(), transl=transl.numpy(),
+        keys=np.array(sorted(ref)), **{f'out_{k}': np.asarray(v) for k, v in ref.items()})
+    print('camera.npz', sorted(ref))
+
+
+def mmi_fixture():
+    """Runs the reference's own mesh_to_mesh_forward (oracle/_ref, built by oracle/build_ref.py; needs a GPU) in a process
+    of its own (oracle/run_ref_mmi.py) on the cases of test_gpu_zz_reference_op.py: the chest-plane queries of the four
+    real bodies, and two seeded random triangle soups (~180 colliding pairs, at most 5 per query).  Stores every collision
+    slot (face index or -1) and the barycentrics of the filled ones."""
+    import subprocess
+    import tempfile
+    t = _test_module('test_gpu_zz_reference_op')
+    rng = np.random.default_rng(11)
+    B, Q, F = 2, 96, 400
+
+    def soup(n, spread, size):
+        c = rng.uniform(-spread, spread, (B, n, 1, 3))
+        return (c + rng.normal(0, size, (B, n, 3, 3))).astype(np.float32)
+    soup_query, soup_target = soup(Q, 1.0, 0.15), soup(F, 1.0, 0.15)
+    out = dict(soup_query=soup_query, soup_target=soup_target)
+    cases = dict(plane=t.plane_queries(G) + (t.PLANE_M,), soup=(soup_query, soup_target, t.SOUP_M))
+    with tempfile.TemporaryDirectory() as tmp:
+        for tag, (query, target, m) in cases.items():
+            inp, outp = os.path.join(tmp, tag + '_in.npz'), os.path.join(tmp, tag + '_out.npz')
+            np.savez(inp, query=query, target=target, max_collisions=np.int64(m))
+            subprocess.run([sys.executable, os.path.join(ROOT, 'oracle', 'run_ref_mmi.py'), inp, outp], check=True, timeout=600)
+            d = np.load(outp)
+            faces = d['faces']
+            assert faces.shape == (query.shape[0], query.shape[1] * m), faces.shape
+            out[f'{tag}_faces'] = faces.astype(np.int32)
+            out[f'{tag}_bcs'] = d['bcs'][faces >= 0].astype(np.float32)
+            print(tag, 'collisions per batch entry', (faces >= 0).sum(1))
+    np.savez_compressed(os.path.join(G, 'ref_mmi.npz'), **out)
+    print('ref_mmi.npz', os.path.getsize(os.path.join(G, 'ref_mmi.npz')), 'bytes')
+
+
 if __name__ == '__main__':
-    which = sys.argv[1:] or ['body', 'smplx', 'head', 'hrnet', 'preprocess', 'b2a', 'p2p', 'v2v']
+    which = sys.argv[1:] or ['body', 'smplx', 'head', 'hrnet', 'preprocess', 'b2a', 'p2p', 'v2v', 'smplx_seed5', 'keypoint',
+                             'camera']
     torch.set_num_threads(8)
     if 'body' in which:
         body_fixture()
@@ -331,3 +436,11 @@ if __name__ == '__main__':
         p2p_fixture()
     if 'v2v' in which:
         v2v_fixture()
+    if 'smplx_seed5' in which:
+        smplx_seed5_fixture()
+    if 'keypoint' in which:
+        keypoint_fixture()
+    if 'camera' in which:
+        camera_fixture()
+    if 'mmi' in which:
+        mmi_fixture()
