@@ -103,6 +103,11 @@ int shapy_smplx_forward(const shapy_smplx_t *m, const float *betas, const float 
 int shapy_smplx_forward_shape(const shapy_smplx_t *m, const float *betas, int batch, float *v_shaped,
                               void *stream);
 
+/* Backward of shapy_smplx_forward_shape: grad_betas (B, num_betas) = shapedirs^T . grad_v_shaped (B,V,3), summed in a
+ * fixed order (a body's result does not depend on its position in the batch). */
+int shapy_smplx_shape_backward(const shapy_smplx_t *m, const float *grad_v_shaped, int batch, float *grad_betas,
+                               void *stream);
+
 /* ------------------------------------------------------- virtual measurements */
 typedef struct {
   int face_idx[5];      /* head_top, left_heel, chest, waist, hips landmark faces */
@@ -121,6 +126,23 @@ int shapy_measure_forward(const float *v_shaped, const int32_t *faces, int batch
 int shapy_measure_forward_tris(const float *triangles, int batch, int num_faces,
                                const shapy_measure_landmarks_t *lm, float *out, float *plane_points,
                                int32_t *plane_counts, int max_points, int32_t *status, void *stream);
+
+/* Backward of shapy_measure_forward: grad_out (B,5) -> grad_v (B,V,3), the first derivative of
+ * sum_j grad_out[b][j] * out[b][j] with the intersection barycentrics and the slicing heights held constant (the
+ * reference computes them under no_grad).  Recomputes the forward's point sets and hulls; no float atomics, so the
+ * result is bit-reproducible.  A NaN circumference with a non-zero grad_out entry makes that body's gradient NaN; a
+ * zero entry contributes nothing.  workspace: shapy_measure_backward_workspace_bytes(num_verts, num_faces) bytes
+ * (the vertex -> face adjacency, rebuilt by every call).  num_verts is limited by the shared-memory staging
+ * (SMPL-X and SMPL fit); beyond it the call fails with SHAPY_ERR_ARG. */
+size_t shapy_measure_backward_workspace_bytes(int num_verts, int num_faces);
+int shapy_measure_backward(const float *v_shaped, const int32_t *faces, int batch, int num_verts, int num_faces,
+                           const shapy_measure_landmarks_t *lm, const float *grad_out, float *grad_v,
+                           void *workspace, size_t workspace_bytes, void *stream);
+
+/* Same on explicit triangles: grad_tris (B,F,3,3), mirroring shapy_measure_forward_tris (and its capacities). */
+int shapy_measure_backward_tris(const float *triangles, int batch, int num_faces,
+                                const shapy_measure_landmarks_t *lm, const float *grad_out, float *grad_tris,
+                                void *stream);
 
 /* Drop-in for mesh_mesh_intersect_cuda.mesh_to_mesh_forward: query (B,Q,3,3), target (B,F,3,3) fp32;
  * collision_faces (B,Q*M) int64 pre-filled by the callee with -1; collision_bcs (B,Q*M,2,3) with 0. */

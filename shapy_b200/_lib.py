@@ -64,10 +64,16 @@ _SIGS = {
     'shapy_smplx_forward': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     'shapy_smplx_forward_shape': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    'shapy_smplx_shape_backward': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     'shapy_measure_forward': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, C.POINTER(MeasureLandmarks), c_void_p,
                                       c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     'shapy_measure_forward_tris': (c_int, [c_void_p, c_int, c_int, C.POINTER(MeasureLandmarks), c_void_p, c_void_p,
                                            c_void_p, c_int, c_void_p, c_void_p]),
+    'shapy_measure_backward_workspace_bytes': (c_size_t, [c_int, c_int]),
+    'shapy_measure_backward': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, C.POINTER(MeasureLandmarks), c_void_p,
+                                       c_void_p, c_void_p, c_size_t, c_void_p]),
+    'shapy_measure_backward_tris': (c_int, [c_void_p, c_int, c_int, C.POINTER(MeasureLandmarks), c_void_p, c_void_p,
+                                            c_void_p]),
     'shapy_mmi_workspace_bytes': (c_size_t, [c_int, c_int, c_int]),
     'shapy_mmi_forward': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                   c_size_t, c_void_p]),

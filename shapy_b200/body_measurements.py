@@ -10,8 +10,42 @@ import os.path as osp
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import ops as _ops
+
+
+class _Measure(torch.autograd.Function):
+    """(B, 5) measurements of `x` = v_shaped (with faces_i32) or triangles, differentiable once in `x`."""
+
+    @staticmethod
+    def forward(ctx, x, faces_i32, landmarks):
+        if faces_i32 is None:
+            out = _ops.measure(landmarks, triangles=x)
+        else:
+            out = _ops.measure(landmarks, v_shaped=x, faces_i32=faces_i32)
+        ctx.landmarks = landmarks
+        ctx.save_for_backward(x, faces_i32)
+        ctx.mark_non_differentiable(out.status)
+        return out, out.status
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out, _grad_status):
+        x, faces_i32 = ctx.saved_tensors
+        if faces_i32 is None:
+            return _ops.measure_backward(ctx.landmarks, grad_out, triangles=x), None, None
+        return _ops.measure_backward(ctx.landmarks, grad_out, v_shaped=x, faces_i32=faces_i32), None, None
+
+
+def _measure(landmarks, x, faces_i32=None):
+    if torch.is_grad_enabled() and x.requires_grad:
+        out, status = _Measure.apply(x, faces_i32, landmarks)
+        out.status = status
+        return out
+    if faces_i32 is None:
+        return _ops.measure(landmarks, triangles=x)
+    return _ops.measure(landmarks, v_shaped=x, faces_i32=faces_i32)
 
 
 class BodyMeasurements(nn.Module):
@@ -79,13 +113,15 @@ class BodyMeasurements(nn.Module):
             raise RuntimeError('BodyMeasurements: intersection-point capacity exceeded; affected values are NaN')
 
     def forward_vertices(self, v_shaped, faces_i32):
-        """Fast path: (B, V, 3) vertices + (F, 3) int32 faces; no (B, F, 3, 3) tensor is materialised."""
-        return self._pack(_ops.measure(self.landmarks(), v_shaped=v_shaped, faces_i32=faces_i32))
+        """Fast path: (B, V, 3) vertices + (F, 3) int32 faces; no (B, F, 3, 3) tensor is materialised.
+        Differentiable once in v_shaped when grad mode is on and it requires grad (see ops.measure_backward)."""
+        return self._pack(_measure(self.landmarks(), v_shaped, faces_i32))
 
     def forward(self, triangles, compute_mass=True, compute_height=True, compute_chest=True, compute_waist=True,
                 compute_hips=True, **kwargs):
-        """triangles: (B, F, 3, 3), as in the reference."""
-        out = self._pack(_ops.measure(self.landmarks(), triangles=triangles))
+        """triangles: (B, F, 3, 3), as in the reference; differentiable once in triangles when grad mode is on and
+        they require grad.  A measurement turned off by its compute_* flag receives no gradient."""
+        out = self._pack(_measure(self.landmarks(), triangles))
         drop = [n for n, f in (('mass', compute_mass), ('height', compute_height), ('chest', compute_chest),
                                ('waist', compute_waist), ('hips', compute_hips)) if not f]
         for n in drop:

@@ -23,7 +23,7 @@ ARCH = ['-gencode', 'arch=compute_100a,code=sm_100a']
 COMMON = ['-O3', '-std=c++17', '-lineinfo', '-Xcompiler', '-fPIC',
           '--expt-relaxed-constexpr']
 # per-file extra flags: the triangle predicates must round like the plain-C oracle
-EXTRA = {'measure.cu': ['-fmad=false'], 'bvh.cu': ['-fmad=false']}
+EXTRA = {'measure.cu': ['-fmad=false'], 'measure_grad.cu': ['-fmad=false'], 'bvh.cu': ['-fmad=false']}
 
 
 def sources():

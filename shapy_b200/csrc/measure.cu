@@ -14,12 +14,10 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "measure.cuh"
 #include "mmi_device.cuh"
 
 namespace shapy {
-
-constexpr int kMaxPts = 512;
-constexpr int kMaxCand = 4096;  // (face, plane, query triangle) candidates that pass the AABB filter, per body
 
 struct MeasureArgs {
   const float *verts;  // (B,V,3) or null
@@ -50,16 +48,6 @@ __device__ __forceinline__ mmi::Tri load_tri(const MeasureArgs &a, int b, int f)
     t.v2 = make_float3(vb[3 * i2], vb[3 * i2 + 1], vb[3 * i2 + 2]);
   }
   return t;
-}
-
-__device__ __forceinline__ bool better_next(double cx, double cz, float ax, float az, float bx, float bz) {
-  // true when candidate b should replace a as the next hull vertex after c (counter-clockwise walk):
-  // b is strictly to the right of c->a, or collinear and farther.
-  double ux = (double)ax - cx, uz = (double)az - cz, wx = (double)bx - cx, wz = (double)bz - cz;
-  double o = ux * wz - uz * wx;
-  if (o < 0) return true;
-  if (o > 0) return false;
-  return (wx * wx + wz * wz) > (ux * ux + uz * uz);
 }
 
 constexpr int kMeasThreads = 512;
@@ -216,21 +204,6 @@ __global__ void __launch_bounds__(kMeasThreads) measure_kernel(MeasureArgs a) {
 //            lengths are summed in chain order, so the result does not depend on timing.
 // Capacity overflows (candidates, points per plane) are reported through `status` AND poison the affected outputs
 // with NaN: a truncated point set must never pass for a measurement.
-constexpr int kM2Threads = 1024;
-constexpr int kM2MaxPts = 1024;
-constexpr int kM2MaxCand = 8192;     // ints; the buffer is reused for the per-chain candidate lists (u16) in phase 3
-constexpr int kM2ChainCap = 640;     // 24 chains x 640 x 2 B = 30 KB <= 32 KB
-
-struct M2Ext { float x, z; int idx; };
-
-__device__ __forceinline__ void m2_key(float x, float z, int k, double &k1, double &k2) {
-  // direction d_k = (dx, dz), k * 45 degrees (unnormalised, exact); tie-break direction = d_k rotated by +90 degrees
-  const int dxs[8] = {1, 1, 0, -1, -1, -1, 0, 1}, dzs[8] = {0, 1, 1, 1, 0, -1, -1, -1};
-  const double dx = dxs[k], dz = dzs[k];
-  k1 = dx * (double)x + dz * (double)z;
-  k2 = -dz * (double)x + dx * (double)z;
-}
-
 __global__ void __launch_bounds__(kM2Threads, 1) measure_smem_kernel(MeasureArgs a) {
   extern __shared__ __align__(16) unsigned char m2_smem[];
   const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;

@@ -385,6 +385,54 @@ __global__ void smplx_shape_kernel_generic(const float *__restrict__ T, const fl
   out[(size_t)b * V3 + c] = v;
 }
 
+// Backward of the T-pose path: grad_betas[b][l] = sum_c S[l][c] grad_v[b][c] for the NB shape rows of the [NC][3V]
+// basis.  A CTA takes SBW bodies x SLW betas: each thread walks the coordinates c = tid, tid + 256, ... (one read of
+// each gradient row, streaming; the basis rows come from L2), then a fixed shuffle tree and a fixed sum over the
+// warps.  A body's result is the same arithmetic wherever it sits in the batch.
+constexpr int SBW = 8, SLW = 10;
+__global__ void __launch_bounds__(256) smplx_shape_backward_kernel(const float *__restrict__ S,
+                                                                   const float *__restrict__ g, int NB, int V3, int B,
+                                                                   float *__restrict__ out) {
+  __shared__ float red[8][SBW * SLW];
+  const int b0 = blockIdx.x * SBW, l0 = blockIdx.y * SLW;
+  const int nb = min(SBW, B - b0), nl = min(SLW, NB - l0);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float acc[SBW][SLW];
+#pragma unroll
+  for (int i = 0; i < SBW; ++i)
+#pragma unroll
+    for (int l = 0; l < SLW; ++l) acc[i][l] = 0.f;
+  for (int c = threadIdx.x; c < V3; c += 256) {
+    float s[SLW];
+#pragma unroll
+    for (int l = 0; l < SLW; ++l) s[l] = l < nl ? __ldg(S + (size_t)(l0 + l) * V3 + c) : 0.f;
+#pragma unroll
+    for (int i = 0; i < SBW; ++i) {
+      if (i < nb) {
+        const float gv = __ldcs(g + (size_t)(b0 + i) * V3 + c);
+#pragma unroll
+        for (int l = 0; l < SLW; ++l) acc[i][l] += gv * s[l];
+      }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < SBW; ++i)
+#pragma unroll
+    for (int l = 0; l < SLW; ++l) {
+      float v = acc[i][l];
+      for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if (lane == 0) red[warp][i * SLW + l] = v;
+    }
+  __syncthreads();
+  for (int j = threadIdx.x; j < SBW * SLW; j += 256) {
+    const int i = j / SLW, l = j % SLW;
+    if (i >= nb || l >= nl) continue;
+    float v = 0.f;
+    for (int w = 0; w < 8; ++w) v += red[w][j];
+    out[(size_t)(b0 + i) * NB + l0 + l] = v;
+  }
+}
+
 template <typename T>
 static T *upload(shapy_smplx *m, const std::vector<T> &h, cudaError_t &err) {
   T *p = nullptr;
@@ -674,6 +722,17 @@ extern "C" int shapy_smplx_forward_shape(const shapy_smplx_t *m, const float *be
     dim3 grid(ceil_div(V3, 256), B);
     smplx_shape_kernel_generic<<<grid, 256, 0, st>>>(d.v_template, d.shapedirs, betas, d.NB, V3, B, v_shaped);
   }
+  SHAPY_LAUNCH_CHECK();
+  return SHAPY_OK;
+}
+
+extern "C" int shapy_smplx_shape_backward(const shapy_smplx_t *m, const float *grad_v_shaped, int B,
+                                          float *grad_betas, void *stream) {
+  SHAPY_REQUIRE(m && grad_v_shaped && grad_betas && B > 0, "shapy_smplx_shape_backward: bad argument");
+  const SmplxDev &d = m->d;
+  dim3 grid(ceil_div(B, SBW), ceil_div(d.NB, SLW));
+  smplx_shape_backward_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d.shapedirs, grad_v_shaped, d.NB, d.V * 3, B,
+                                                                      grad_betas);
   SHAPY_LAUNCH_CHECK();
   return SHAPY_OK;
 }

@@ -14,6 +14,7 @@ from collections import defaultdict
 import numpy as np
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from .... import ops as _ops
 from .utils import KeypointTensor, find_joint_kin_chain, to_tensor
@@ -52,6 +53,18 @@ def _keypoint_names(num):
         pass
     names = list(SMPLX_BODY_JOINT_NAMES)
     return (names + [f'keypoint_{i:03d}' for i in range(len(names), num)])[:max(num, 0)]
+
+
+class _ShapeBlend(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, betas, model):
+        ctx.model = model
+        return _ops.smplx_forward_shape(model, betas)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_v_shaped):
+        return _ops.smplx_shape_backward(ctx.model, grad_v_shaped), None
 
 
 class SMPLX(nn.Module):
@@ -211,7 +224,13 @@ class SMPLX(nn.Module):
 
     # ------------------------------------------------------------------ forward
     def forward_shape(self, betas=None):
-        v_shaped = _ops.smplx_forward_shape(self.packed(betas.device), betas)
+        """v_shaped = v_template + shapedirs . betas; differentiable once in betas when grad mode is on and betas
+        require grad."""
+        model = self.packed(betas.device)
+        if torch.is_grad_enabled() and betas.requires_grad:
+            v_shaped = _ShapeBlend.apply(betas, model)
+        else:
+            v_shaped = _ops.smplx_forward_shape(model, betas)
         return {'vertices': v_shaped, 'betas': betas, 'v_shaped': v_shaped}
 
     def forward(self, global_rot=None, body_pose=None, left_hand_pose=None, right_hand_pose=None, jaw_pose=None,

@@ -160,6 +160,20 @@ def smplx_forward_shape(model: SmplxModel, betas) -> torch.Tensor:
     return out
 
 
+def smplx_shape_backward(model: SmplxModel, grad_v_shaped) -> torch.Tensor:
+    """(B, V, 3) gradient of v_shaped -> (B, num_betas) gradient of betas (backward of smplx_forward_shape)."""
+    g = _cuda_f32(grad_v_shaped, 'grad_v_shaped')
+    B = g.shape[0]
+    if g.shape != (B, model.V, 3):
+        raise RuntimeError(f'grad_v_shaped must be ({B}, {model.V}, 3), got {tuple(g.shape)}')
+    out = torch.empty(B, model.NB, dtype=torch.float32, device=g.device)
+    if B == 0:
+        return out
+    with torch.cuda.device(g.device):
+        check(lib().shapy_smplx_shape_backward(model.handle, ptr(g), B, ptr(out), stream_ptr()), 'smplx_shape_backward')
+    return out
+
+
 # ------------------------------------------------------------------------------------ measurements
 def make_landmarks(lm: dict) -> _lib.MeasureLandmarks:
     """lm: {'head_top','left_heel','chest','waist','hips'} -> {'face_idx', 'bc'}."""
@@ -213,6 +227,40 @@ def measure(landmarks: _lib.MeasureLandmarks, v_shaped=None, faces_i32=None, tri
     if return_points:
         return out, pts, cnt, status
     return out
+
+
+def measure_backward(landmarks: _lib.MeasureLandmarks, grad_out, v_shaped=None, faces_i32=None, triangles=None):
+    """Backward of `measure`: grad_out (B, 5) -> the gradient of v_shaped (B, V, 3) or of triangles (B, F, 3, 3).
+
+    First derivative only, with the intersection barycentrics and the slicing heights held constant.  Where `measure`
+    returned a NaN circumference, the body's gradient is NaN if its grad_out entry is non-zero; a zero entry
+    contributes nothing."""
+    g = _cuda_f32(grad_out, 'grad_out')
+    if triangles is not None:
+        x = _cuda_f32(triangles, 'triangles')
+        B, F = x.shape[0], x.shape[1]
+    else:
+        x = _cuda_f32(v_shaped, 'v_shaped')
+        B, V = x.shape[0], x.shape[1]
+        if not (torch.is_tensor(faces_i32) and faces_i32.is_cuda and faces_i32.dtype == torch.int32):
+            raise RuntimeError('faces_i32 must be a CUDA int32 tensor')
+        faces_i32 = faces_i32.contiguous()
+        F = faces_i32.shape[0]
+    if g.shape != (B, 5):
+        raise RuntimeError(f'grad_out must be ({B}, 5), got {tuple(g.shape)}')
+    dev = x.device
+    grad = torch.empty_like(x)
+    if B == 0:
+        return grad
+    with torch.cuda.device(dev):
+        if triangles is not None:
+            check(lib().shapy_measure_backward_tris(ptr(x), B, F, C.byref(landmarks), ptr(g), ptr(grad),
+                                                    stream_ptr()), 'measure_backward')
+        else:
+            ws = _WS.get('measure_bwd', lib().shapy_measure_backward_workspace_bytes(V, F), dev)
+            check(lib().shapy_measure_backward(ptr(x), ptr(faces_i32), B, V, F, C.byref(landmarks), ptr(g), ptr(grad),
+                                               ptr(ws), ws.numel(), stream_ptr()), 'measure_backward')
+    return grad
 
 
 def mesh_to_mesh_forward(query_triangles, target_triangles, max_collisions=16, print_timings=False):

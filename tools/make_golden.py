@@ -28,6 +28,8 @@ Everything written here is a small fixture that travels to the GPU box, where
   camera.npz            the reference weak_persp_to_blender (demo.py) on seeded targets and camera parameters
   ref_mmi.npz           the reference mesh_to_mesh_forward kernel (oracle/_ref; `python tools/make_golden.py mmi` on a
                         GPU) on the cases of test_gpu_zz_reference_op.py
+  measure_grad.npz      gradients of the reference's BodyMeasurements under autograd (its mesh_mesh_intersection module
+                        replaced by the C restatement oracle/mmi_oracle.c) on the four bodies of img00_body.npz
 """
 import hashlib
 import json
@@ -416,6 +418,77 @@ def mmi_fixture():
     print('ref_mmi.npz', os.path.getsize(os.path.join(G, 'ref_mmi.npz')), 'bytes')
 
 
+
+def measure_grad_fixture():
+    """The reference's body_measurements.py loaded verbatim, its CUDA collision module replaced by
+    oracle.measure_oracle.mesh_to_mesh_forward (the C restatement of op.cu the golden measurements pin), run under
+    autograd on the four bodies of img00_body.npz.  Each measurement's gradient with respect to v_shaped is stored
+    on its own: mass dense for bodies 0 and 1 (it touches every vertex), height and the circumferences sparse as
+    (body, vertex) indices + values.  The mass gradient is the reference's compute_mass differentiated in float64: in
+    float32 its autograd loses ~1e-5 of max|grad| to cancellation between the faces around a vertex."""
+    import importlib.util
+    import types
+    from oracle import measure_oracle
+    mmi = types.ModuleType('mesh_mesh_intersection')
+
+    class MeshMeshIntersection(torch.nn.Module):
+        def __init__(self, max_collisions=16):
+            super().__init__()
+            self.max_collisions = max_collisions
+
+        def forward(self, query, target):
+            f, b = measure_oracle.mesh_to_mesh_forward(query.detach().numpy(), target.detach().numpy(),
+                                                       self.max_collisions)
+            return torch.from_numpy(f), torch.from_numpy(b)
+    mmi.MeshMeshIntersection = MeshMeshIntersection
+    saved = sys.modules.get('mesh_mesh_intersection')
+    sys.modules['mesh_mesh_intersection'] = mmi
+    try:
+        R = os.path.join(REF, 'mesh-mesh-intersection')
+        spec = importlib.util.spec_from_file_location('ref_body_measurements',
+                                                      os.path.join(R, 'body_measurements', 'body_measurements.py'))
+        bm = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(bm)
+        module = bm.BodyMeasurements({'meas_definition_path': os.path.join(R, 'data', 'measurement_defitions.yaml'),
+                                      'meas_vertices_path': os.path.join(R, 'data', 'smplx_measurements.yaml')})
+    finally:
+        if saved is None:
+            sys.modules.pop('mesh_mesh_intersection', None)
+        else:
+            sys.modules['mesh_mesh_intersection'] = saved
+    g = np.load(os.path.join(G, 'img00_body.npz'))
+    bodies = np.concatenate([g['v_shaped'][None], g['extra_v_shaped']], 0).astype(np.float32)
+    faces = torch.from_numpy(g['faces'].astype(np.int64))
+    out = dict(values=np.zeros((len(bodies), 5), np.float32))
+    names = ('mass', 'height', 'chest', 'waist', 'hips')
+    sparse = {n: ([], [], []) for n in names[1:]}
+    mass = []
+    for b, v in enumerate(bodies):
+        vs = torch.from_numpy(v)[None].requires_grad_(True)
+        meas = module(vs[:, faces])['measurements']
+        for i, n in enumerate(names):
+            val = meas[n]['tensor']
+            out['values'][b, i] = float(val[0].detach())
+            grad, = torch.autograd.grad(val.sum(), vs, retain_graph=i < 4)
+            grad = grad[0].numpy()
+            if n == 'mass':
+                if b < 2:
+                    v64 = torch.from_numpy(v).double()[None].requires_grad_(True)
+                    mass.append(torch.autograd.grad(module.compute_mass(v64[:, faces]).sum(), v64)[0][0].numpy())
+                continue
+            idx = np.where(np.abs(grad).sum(-1) > 0)[0]
+            sparse[n][0].append(np.full(len(idx), b, np.int32))
+            sparse[n][1].append(idx.astype(np.int32))
+            sparse[n][2].append(grad[idx].astype(np.float32))
+        print('body', b, dict(zip(names, out['values'][b])))
+    out['mass_grad'] = np.stack(mass).astype(np.float32)
+    for n, (bb, idx, val) in sparse.items():
+        out[f'{n}_body'], out[f'{n}_vertex'], out[f'{n}_grad'] = map(np.concatenate, (bb, idx, val))
+        print(n, 'non-zero vertices per body', np.bincount(out[f'{n}_body'], minlength=len(bodies)))
+    np.savez_compressed(os.path.join(G, 'measure_grad.npz'), **out)
+    print('measure_grad.npz', os.path.getsize(os.path.join(G, 'measure_grad.npz')), 'bytes')
+
+
 if __name__ == '__main__':
     which = sys.argv[1:] or ['body', 'smplx', 'head', 'hrnet', 'preprocess', 'b2a', 'p2p', 'v2v', 'smplx_seed5', 'keypoint',
                              'camera']
@@ -444,3 +517,5 @@ if __name__ == '__main__':
         camera_fixture()
     if 'mmi' in which:
         mmi_fixture()
+    if 'measure_grad' in which:
+        measure_grad_fixture()
